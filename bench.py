@@ -9,10 +9,13 @@ Default config = c2, BASELINE.json's headline: ProcessorParseRegexNative, nginx 
 rank parses its own shard, no collective on the data path.  One "step" = one pass of the hot path over the whole batch.
 
   value      input MB/s (1 MB = 1e6 B of log bytes, separators included) with the batch resident in HBM.  Timing: after
-             W >= 3 warm-up steps the timed region holds R rounds of exactly K steps, each round bracketed by CUDA events
-             on the engine's stream, R sized so that the region lasts >= 1 s; the whole region sits between barrier +
-             synchronize on both sides.  ms_per_step = MEDIAN round / K (min also reported), value = sum of the shard
-             bytes / max over ranks of that time.
+             a warm-up that keeps the device busy for the 1.2 s the clock sampler needs and ends with W >= 3 steps
+             back to back between two CUDA events, the timed region holds exactly K steps (--steps; by default sized
+             from the step time of those W with a 10 % margin, so that it lasts >= 1 s), split into up to 20 chunks
+             of >= 10 ms, each between two CUDA events on the engine's stream.  One more warm-up step is queued right
+             ahead of the region, which sits between barrier + synchronize on both sides.
+             ms_per_step = MEDIAN over the chunks of chunk time / its steps (min also reported), value = sum of the
+             shard bytes / max over ranks of that time.
   e2e        the same metric through the reference-facing C-ABI call of the path with HOST buffers (pinned arena in,
              result tables out), H2D and D2H inside the timed region -- what the engine contributes to a pipeline.
   e2e_plugin (c2) one level up: ProcessorInstance::Process(std::vector<PipelineEventGroup>&) of the B200-backed
@@ -21,6 +24,10 @@ rank parses its own shard, no collective on the data path.  One "step" = one pas
              event-object model (one heap LogEvent per line, one AddLog per capture) costs more than the parsing
              itself on either arm; cpu_baseline is measured at the same boundary with the same model.
   roofline   achieved = algorithmic bytes of SURVEY.md section 8(d) per step / median device time of one step.
+
+  --dump-outputs DIR writes the result tables of the last timed step (rank 0) as DIR/<name>.npy, see dump_outputs();
+  c5 calls the engine once per sub-batch of 1 Mi lines into the same tables, so only its last call's tables are written.
+  The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -39,13 +46,19 @@ sys.path.insert(0, ROOT)
 
 UNIT = "MB/s"
 GROUP_BYTES = 512 * 1024  # LogFileReader.cpp:97: the reader hands the processors groups of at most 512 KB
-TIMED_REGION_S = 1.0
+REGION_S = 1.0  # timed region without --steps: at least this long
+CHUNK_MS = 10.0  # timed steps between two CUDA events: at least this long (an event costs ~2 us on a B200)
+MAX_CHUNKS = 20
+DUMP_BYTES = 64 * 10 ** 6  # --dump-outputs: all files together
+DUMP_SEED = 20261017  # --dump-outputs: the row sample of tables larger than DUMP_BYTES
 
 
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=30)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default: enough for a region of >= %g s, sized from the warm-up's step time; "
+                         "the reference arm: 30)" % REGION_S)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="c2", choices=["c1", "c2", "c3", "c4", "c5"])
@@ -53,8 +66,13 @@ def parse_args():
     ap.add_argument("--e2e", default="auto", choices=["auto", "plugin", "abi", "none"])
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--region-s", type=float, default=TIMED_REGION_S)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result tables of the last timed step as DIR/<name>.npy (float64; c5: only "
+                         "those of the step's last engine call, up to %d lines)" % C5.SUB)
+    args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def dist_env():
@@ -240,6 +258,24 @@ def _vp(a):
     return a.ctypes.data_as(ctypes.c_void_p)
 
 
+def dump_outputs(cfg, out_dir):
+    """Writes the tables the timed path returned in its last step (cfg.outputs(): name -> array) as out_dir/<name>.npy
+    in float64, which holds every u8 / u32 value exactly.  If the tables with the most rows would take the files past
+    DUMP_BYTES, each of them keeps the same DUMP_SEED-seeded sample of rows, whose row numbers go to rows.npy."""
+    outs = {k: np.asarray(a) for k, a in cfg.outputs().items()}
+    n = max(a.shape[0] for a in outs.values())
+    per_row = sum(a.size // n for a in outs.values() if a.shape[0] == n)
+    fixed = sum(a.size for a in outs.values() if a.shape[0] != n)
+    m = min(n, (DUMP_BYTES // 8 - 1024 - fixed) // (per_row + 1))  # 1024 values of room for the .npy headers
+    if m < n:
+        rows = np.sort(np.random.default_rng(DUMP_SEED).choice(n, m, replace=False))
+        outs = {k: a[rows] if a.shape[0] == n else a for k, a in outs.items()}
+        outs["rows"] = rows
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in outs.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a.astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------------------ CPU arms (oracle)
 def cpu_threads_run(work, threads):
     t0 = time.perf_counter()
@@ -390,6 +426,9 @@ class C2(Config):
         return (self.d_status.cpu().numpy(), self.d_co.cpu().numpy().view(np.uint32).reshape(n, G),
                 self.d_cl.cpu().numpy().view(np.uint32).reshape(n, G))
 
+    def outputs(self):
+        return dict(zip(("status", "cap_off", "cap_len"), self.results()))
+
     def check(self):
         """every row of a bounded prefix against the CPU oracle (rank 0)"""
         from loongcollector_b200 import synth
@@ -515,6 +554,10 @@ class C1(Config):
         self.got = self.eng.split_lines_dev(self.d_buf.data_ptr(), self.in_bytes, 10, self.d_off.data_ptr(),
                                             self.d_len.data_ptr(), self.n + 16)
 
+    def outputs(self):
+        return {"line_count": np.array([self.got]), "line_off": self.d_off[:self.got].cpu().numpy().view(np.uint32),
+                "line_len": self.d_len[:self.got].cpu().numpy().view(np.uint32)}
+
     def check(self):
         from oracle import oracle as orc
         assert self.got == self.n
@@ -610,6 +653,12 @@ class C3(Config):
         self.got, self.ctr = self.eng.multiline_split_dev(self.d_buf.data_ptr(), self.in_bytes, self.start, None, None,
                                                           False, self.o.data_ptr(), self.l.data_ptr(),
                                                           self.f.data_ptr(), self.cap)
+
+    def outputs(self):
+        return {"record_count": np.array([self.got]), "counters": np.array([int(x) for x in self.ctr]),
+                "record_off": self.o[:self.got].cpu().numpy().view(np.uint32),
+                "record_len": self.l[:self.got].cpu().numpy().view(np.uint32),
+                "record_flags": self.f[:self.got].cpu().numpy()}
 
     def check(self):
         from loongcollector_b200 import synth
@@ -728,6 +777,16 @@ class C4(Config):
                                  self.tl.data_ptr())
         self.eng.regex_parse_dev(self.rx, self.d_buf.data_ptr(), self.in_bytes, self.to.data_ptr(), self.tl.data_ptr(),
                                  n, self.G, self.rs.data_ptr(), self.rco.data_ptr(), self.rcl.data_ptr())
+
+    def outputs(self):
+        """the tables lc_delim_regex_chain returns"""
+        n, MF, G = self.n, self.MF, self.G
+
+        def u32(t, w):
+            return t.view(n, w).cpu().numpy().view(np.uint32)
+        return {"status": self.st.cpu().numpy(), "nfields": self.nf.cpu().numpy().view(np.uint32),
+                "field_off": u32(self.fo, MF), "field_len": u32(self.fl, MF), "field_dq": u32(self.fd, MF),
+                "re_status": self.rs.cpu().numpy(), "cap_off": u32(self.rco, G), "cap_len": u32(self.rcl, G)}
 
     def finish_setup(self):
         n, MF = self.n, self.MF
@@ -897,6 +956,12 @@ class C5(Config):
         for s in range(self.nsub):
             self.run_sub(s)
 
+    def outputs(self):
+        """the tables of the step's last call (the calls share them)"""
+        return {"which": self.d_wh.cpu().numpy(), "status": self.d_st.cpu().numpy(),
+                "cap_off": self.d_co.cpu().numpy().view(np.uint32).reshape(self.sub, self.GP),
+                "cap_len": self.d_cl.cpu().numpy().view(np.uint32).reshape(self.sub, self.GP)}
+
     def check(self):
         """every row of the LAST sub-batch against the oracle: per-pattern PCRE2 results on the pool lines, merged
         first-match-wins and expanded through the sampling index"""
@@ -1012,7 +1077,7 @@ def run_reference(args):
         from loongcollector_b200 import synth
         n = args.lines or 4 * 1024 * 1024
         buf, off, ln = make_workload(n, shard_seed(0))
-        reps = max(1, args.steps)
+        reps = args.steps or 30
         for _ in range(min(args.warmup, 2)):
             cpu_regex_parse(synth.NGINX_PATTERN, len(synth.NGINX_KEYS), buf, off, ln, cores)
         ts = np.array([cpu_regex_parse(synth.NGINX_PATTERN, len(synth.NGINX_KEYS), buf, off, ln, cores)[0]
@@ -1039,7 +1104,7 @@ def run_reference(args):
         cfg.setup_host()
         for _ in range(min(args.warmup, 1)):
             cfg.cpu_baseline()
-        res = [cfg.cpu_baseline() for _ in range(max(1, args.steps))]
+        res = [cfg.cpu_baseline() for _ in range(args.steps or 30)]
         vals = np.array([r["value"] for r in res])
         v = float(np.median(vals))
         sample = res[0]["sample"]
@@ -1085,47 +1150,56 @@ def run_ours(args):
             dist.barrier()
         torch.cuda.synchronize()
 
-    K = max(1, args.steps)
     W = max(args.warmup, 3)
     sampler = ClockSampler(local_rank)
     sampler.start()  # >= 1 s before the timed region: the first samples of nvidia-smi -lms are slow to arrive
     t_sampler = time.time()
-    # ---- warm-up, timed to size the region
+    # ---- warm-up: the device kept busy until the sampler has run for 1.2 s, then W steps back to back between two
+    # CUDA events, whose time per step sizes the default K and the chunks
+    warm = 0
+    w0, w1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     with torch.cuda.stream(stream):
+        while time.time() - t_sampler < 1.2:
+            cfg.step()
+            torch.cuda.synchronize()
+            warm += 1
+        w0.record(stream)
         for _ in range(W):
             cfg.step()
+        w1.record(stream)
     torch.cuda.synchronize()
-    if hasattr(cfg, "finish_setup"):
-        cfg.finish_setup()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    with torch.cuda.stream(stream):
-        e0.record(stream)
-        for _ in range(3):
-            cfg.step()
-        e1.record(stream)
-    torch.cuda.synchronize()
-    est_ms = max(e0.elapsed_time(e1) / 3, 1e-3)
-    rounds = int(min(400, max(5, np.ceil(args.region_s * 1e3 / (est_ms * K)))))
-    if world > 1:  # same number of rounds everywhere
-        t = torch.tensor([rounds], dtype=torch.int64, device=dev)
+    warm += W
+    step_ms = w0.elapsed_time(w1) / W
+    # the warm-up's steps run up to a few % slower than the region's: sized for 10 % more than REGION_S
+    K = args.steps or int(np.ceil(1.1 * REGION_S * 1e3 / step_ms))
+    if world > 1 and not args.steps:  # the same K everywhere
+        t = torch.tensor([K], dtype=torch.int64, device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        rounds = int(t.item())
-    time.sleep(max(0.0, 1.2 - (time.time() - t_sampler)))
-    ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(rounds)]
+        K = int(t.item())
+    # the K steps in chunks of >= CHUNK_MS between CUDA events, for a median / min / max over the chunks
+    n_chunks = max(1, min(MAX_CHUNKS, K, int(K * step_ms // CHUNK_MS)))
+    bounds = [K * i // n_chunks for i in range(n_chunks + 1)]
+    ev = [torch.cuda.Event(enable_timing=True) for _ in bounds]
     barrier()
     sampler.mark_region()
-    launches0 = eng.launches
     with torch.cuda.stream(stream):
-        for r in range(rounds):
-            ev[r][0].record(stream)
-            for _ in range(K):
+        cfg.step()  # one more warm-up step, queued right ahead: the region starts on a busy device
+        warm += 1
+        launches0 = eng.launches
+        ev[0].record(stream)
+        for i in range(n_chunks):
+            for _ in range(bounds[i + 1] - bounds[i]):
                 cfg.step()
-            ev[r][1].record(stream)
+            ev[i + 1].record(stream)
     barrier()
     clocks = sampler.stop()
     launches_total = eng.launches - launches0
-    per_step = np.array([a.elapsed_time(b) for a, b in ev]) / K
+    per_step = np.array([a.elapsed_time(b) for a, b in zip(ev[:-1], ev[1:])]) / np.diff(bounds)
     med, mn, mx = float(np.median(per_step)), float(per_step.min()), float(per_step.max())
+    if hasattr(cfg, "finish_setup"):
+        cfg.finish_setup()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(cfg, args.dump_outputs)
     value, ms_per_step = job_throughput(cfg.in_bytes, med, world, dev)
     value_best, _ = job_throughput(cfg.in_bytes, mn, world, dev)
     per_rank = gather_rank_stats([mn, med, mx], world, dev)
@@ -1211,13 +1285,14 @@ def run_ours(args):
     if rank == 0:
         out = {
             "metric": cfg.metric, "value": value, "unit": UNIT, "n_gpus": world, "steps": K,
-            "warmup": W, "ms_per_step": ms_per_step, "higher_is_better": True, "scaling": "weak",
+            "warmup": warm, "ms_per_step": ms_per_step, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "u8", "data": "synthetic",
             "config": {"workload": cfg.workload(), "units_per_gpu": cfg.units, "bytes_per_gpu": cfg.in_bytes,
                        "l2": "inputs (%.0f MB per GPU) larger than L2, no flush" % (cfg.in_bytes / 1e6),
                        **cfg.extra},
-            "timing": {"statistic": "median over rounds of (CUDA-event time of K steps) / K, max over ranks",
-                       "rounds": rounds, "timed_region_s": float(per_step.sum() * K / 1e3),
+            "timing": {"statistic": "median over chunks of the K steps of (CUDA-event time of the chunk / its steps), "
+                                    "max over ranks",
+                       "chunks": n_chunks, "timed_region_s": float((per_step * np.diff(bounds)).sum() / 1e3),
                        "ms_per_step_min": mn, "ms_per_step_max": mx, "value_at_min": value_best,
                        "per_rank_ms_per_step_min_med_max": per_rank},
             "lines_per_s": total_units / (ms_per_step * 1e-3),
@@ -1226,7 +1301,7 @@ def run_ours(args):
                          "algorithmic_bytes_per_step": cfg.alg_bytes, "kernel": cfg.dominant,
                          "kernel_ms": ms_per_step},
             "cpu_baseline": cpu, "e2e": e2e, "gpu_launches": int(launches_total),
-            "gpu_launches_per_step": launches_total / float(rounds * K), "clocks": clocks, "host_placement": placement,
+            "gpu_launches_per_step": launches_total / float(K), "clocks": clocks, "host_placement": placement,
         }
         if e2e_plugin is not None:
             out["e2e_plugin"] = e2e_plugin

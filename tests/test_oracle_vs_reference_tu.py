@@ -1,34 +1,65 @@
 """The oracle's delimiter FSM restatement checked against the REFERENCE's own translation unit
-(core/parser/DelimiterModeFsmParser.cpp compiled in place by oracle/build_ref.sh into oracle/_ref/)."""
+(core/parser/DelimiterModeFsmParser.cpp).  What that translation unit returns for every input below is stored in
+tests/golden/ref_delim_fsm.npz (recorded by tests/golden/extract_delim_fsm_vectors.py from oracle/_ref/, which
+oracle/build_ref.sh compiles in place from a reference checkout), so the comparison runs without one."""
 import ctypes as C
+import hashlib
 import os
 import random
 
 import numpy as np
-import pytest
 
 from oracle import oracle as orc
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SO = os.path.join(ROOT, "oracle", "_ref", "libref_delim.so")
-
-pytestmark = pytest.mark.skipif(not os.path.exists(SO), reason="oracle/_ref not built (needs /root/reference)")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_delim_fsm.npz")
+N_RANDOM = 80000
 
 
-def ref_fsm(lib, line: bytes, sep: int, quote: int):
-    out = np.zeros(len(line) * 5 + 64, np.uint8)
-    used = C.c_uint64(0)
-    k = lib.ref_delim_fsm(line, 0, len(line), C.c_char(bytes([sep])), C.c_char(bytes([quote])),
-                          out.ctypes.data_as(C.c_void_p), out.size, C.byref(used))
-    if k < 0:
-        return None
-    cols, at = [], 0
-    raw = out.tobytes()
-    for _ in range(k):
-        l = int.from_bytes(raw[at:at + 4], "little")
-        cols.append(raw[at + 4:at + 4 + l])
-        at += 4 + l
-    return cols
+def fsm_cases():
+    """(line, sep, quote) in a fixed order: N_RANDOM seeded random lines over small alphabets dense in separators and
+    quotes, then the reference's own TestProcessDoubleQuote inputs (ProcessorParseDelimiterNativeUnittest.cpp:1841-1904)."""
+    rng = random.Random(20260922)
+    for sep, quote in ((44, 39), (44, 34), (124, 39), (9, 34)):
+        alpha = "ab1 " + chr(sep) * 3 + chr(quote) * 3 + "x,"
+        for _ in range(N_RANDOM // 4):
+            yield "".join(rng.choice(alpha) for _ in range(rng.randint(1, 24))).encode(), sep, quote
+    for url in ("''PutData?Category=YunOsAccountOpLog", "PutData?Category=YunOs''AccountOpLog",
+                "PutData?Category=YunOsAccountOpLog''", "''PutData?Category=YunOsAccountOpLog'",
+                "'PutData?Category=Yun'Os'AccountOpLog'", "'PutData?Category=YunOs''AccountOpLog'",
+                "'PutData?Category=YunOsAccountOpLog''", "'''PutData?Category=YunOs''AccountOpLog'''"):
+        yield ("2013-10-31 21:03:49,POST," + url + ",0.024").encode(), 44, 39
+
+
+def cases_digest(cases):
+    h = hashlib.sha256()
+    for line, sep, quote in cases:
+        h.update(len(line).to_bytes(4, "little") + line + bytes([sep, quote]))
+    return h.hexdigest()
+
+
+def encode_results(results):
+    """Column lists (None = the FSM rejects the line) -> the arrays stored in ref_delim_fsm.npz."""
+    ncols = np.array([-1 if r is None else len(r) for r in results], np.int16)
+    col_len = np.array([len(c) for r in results if r for c in r], np.uint32)
+    col_bytes = np.frombuffer(b"".join(c for r in results if r for c in r), np.uint8)
+    return {"ncols": ncols, "col_len": col_len, "col_bytes": col_bytes}
+
+
+def decode_results(ncols, col_len, col_bytes):
+    raw = col_bytes.tobytes()
+    out, j, at = [], 0, 0
+    for k in ncols.tolist():
+        if k < 0:
+            out.append(None)
+            continue
+        cols = []
+        for l in col_len[j:j + k].tolist():
+            cols.append(raw[at:at + l])
+            at += l
+        out.append(cols)
+        j += k
+    assert j == col_len.size and at == len(raw)
+    return out
 
 
 def oracle_fsm(line: bytes, sep: int, quote: int):
@@ -54,25 +85,14 @@ def oracle_fsm(line: bytes, sep: int, quote: int):
 
 
 def test_fsm_restatement_equals_reference_translation_unit():
-    lib = C.CDLL(SO)
-    lib.ref_delim_fsm.restype = C.c_int64
-    lib.ref_delim_fsm.argtypes = [C.c_char_p, C.c_int32, C.c_int32, C.c_char, C.c_char, C.c_void_p, C.c_uint64,
-                                  C.POINTER(C.c_uint64)]
-    rng = random.Random(20260922)
-    n = fails = 0
-    for sep, quote in ((44, 39), (44, 34), (124, 39), (9, 34)):
-        alpha = "ab1 " + chr(sep) * 3 + chr(quote) * 3 + "x,"
-        for _ in range(20000):
-            line = "".join(rng.choice(alpha) for _ in range(rng.randint(1, 24))).encode()
-            r, o = ref_fsm(lib, line, sep, quote), oracle_fsm(line, sep, quote)
-            assert r == o, (line, sep, quote, r, o)
-            n += 1
-            fails += r is None
-    assert n == 80000 and 1000 < fails < n - 1000  # both outcomes exercised
-    # the reference's own TestProcessDoubleQuote inputs (ProcessorParseDelimiterNativeUnittest.cpp:1841-1904)
-    for url in ("''PutData?Category=YunOsAccountOpLog", "PutData?Category=YunOs''AccountOpLog",
-                "PutData?Category=YunOsAccountOpLog''", "''PutData?Category=YunOsAccountOpLog'",
-                "'PutData?Category=Yun'Os'AccountOpLog'", "'PutData?Category=YunOs''AccountOpLog'",
-                "'PutData?Category=YunOsAccountOpLog''", "'''PutData?Category=YunOs''AccountOpLog'''"):
-        line = ("2013-10-31 21:03:49,POST," + url + ",0.024").encode()
-        assert ref_fsm(lib, line, 44, 39) == oracle_fsm(line, 44, 39), url
+    cases = list(fsm_cases())
+    with np.load(GOLDEN) as g:
+        assert str(g["cases_sha256"]) == cases_digest(cases), "inputs differ from those the vectors were recorded on"
+        want = decode_results(g["ncols"], g["col_len"], g["col_bytes"])
+    assert len(want) == len(cases) == N_RANDOM + 8
+    fails = 0
+    for n, ((line, sep, quote), r) in enumerate(zip(cases, want)):
+        o = oracle_fsm(line, sep, quote)
+        assert r == o, (line, sep, quote, r, o)
+        fails += n < N_RANDOM and r is None
+    assert 1000 < fails < N_RANDOM - 1000  # both outcomes exercised

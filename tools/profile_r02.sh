@@ -6,7 +6,7 @@
 TAG=${1:-r02}
 CONFIGS=${2:-"c1 c2 c3 c4 c5"}   # optional: only these configs
 mkdir -p gpurun_out
-B="python bench.py --steps 2 --warmup 3 --region-s 0.01 --no-e2e --no-cpu-baseline"
+B="python bench.py --steps 2 --warmup 3 --no-e2e --no-cpu-baseline"
 for c in $CONFIGS; do
   L=""; [ $c = c5 ] && L="--lines 2097152"
   timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv \
